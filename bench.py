@@ -11,12 +11,17 @@ One JSON line.  What it holds (BASELINE.json: "instances/sec (predict_instances 
                                 in HBM; `e2e` = host image in -> host labels + polygons out through the public API.
                                 N > 1: every rank processes its own copy of the image (weak scaling, no data-path collective).
   value_3d / e2e_3d / roofline_3d   configs[2]: StarDist3D.predict_instances on a 128x512x512 volume, Rays_GoldenSpiral(96),
-                                default Config3D; same two timings (fewer steps, stated in config.steps_3d).
+                                default Config3D; same two timings over the same number of steps.
   big_2d / big_3d               configs[3] / [4]: predict_instances_big on a tiled 8192x8192 image / a 512^3 anisotropic volume,
                                 blocks sharded over the N ranks (strong scaling: the image is fixed, value = instances of the
                                 whole image / max-over-ranks wall time incl. the device-to-device tile gather and the D2H of
                                 the assembled label map on rank 0).
   cpu_baseline                  the reference's CPU path timed on this box's host cores (see --impl reference).
+
+--steps K sets the timed steps of configs[1] and configs[2]; the predict_instances_big runs of configs[3] / [4] are timed
+over fixed passes (2 for the image, 1 for the volume, each after one warm-up pass).  --dump-outputs DIR writes what the
+last timed step of configs[1] / [2] returned, as float32 / float64 .npy files; of the 3-D label volume only the voxels at
+dump_voxels_3d() are written.
 """
 import argparse, json, os, sys, time, threading, subprocess
 import numpy as np
@@ -36,6 +41,14 @@ BIG_2D = dict(shape=(8192, 8192), block_size=2304, min_overlap=128, context=96)
 BIG_3D = dict(shape=(512, 512, 512), block_size=304, min_overlap=32, context=32, anisotropy=(2, 1, 1))
 REF_SAMPLE_3D = (64, 256, 256)     # CPU arms time one eighth of the 3-D volume per step (bounded sample; instances/s is intensive)
 METRIC = "instances/sec (predict_instances end-to-end)"
+DUMP_LIMIT = 64 << 20          # bytes written by --dump-outputs at most
+
+
+def dump_voxels_3d(n):
+    """flat indices of the voxels of the 3-D label volume that --dump-outputs writes (labels_3d_sample.npy): a fixed sample"""
+    return np.sort(np.random.default_rng(0).choice(n, 1 << 21, replace=False))
+
+
 W2D = "StarDist2D predict_instances, 1024x1024, n_rays=32, seeded synthetic U-Net weights (configs[1])"
 W3D = "StarDist3D predict_instances, 128x512x512, Rays_GoldenSpiral n_rays=96, seeded synthetic U-Net weights (configs[2])"
 
@@ -209,7 +222,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the 2-D and the 3-D workload (device and e2e timing each); the big-image runs use fixed passes")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -217,6 +231,8 @@ def main():
     ap.add_argument("--skip-big", action="store_true")
     ap.add_argument("--dim", type=int, default=2)          # reference-worker only
     ap.add_argument("--threads", type=int, default=8)      # reference-worker only
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the 2-D and the 3-D workload returned as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -253,8 +269,9 @@ def main():
               ("cand_end", "nms_end", "nms"), ("nms_end", "label_end", "coord_label"))
 
     def time_device(model, x_dev, shape, pthr, nthr, steps):
-        """device-resident timing: CUDA events around predict_instances_device, L2 flushed between steps"""
-        n_inst = 0; dev_ms = 0.0; stage = {}; n_cand = 0
+        """device-resident timing: CUDA events around predict_instances_device, L2 flushed between steps;
+        also returns what the last step computed"""
+        n_inst = 0; dev_ms = 0.0; stage = {}; n_cand = 0; last = None
         for _ in range(steps):
             flush.zero_()
             model._events = []
@@ -266,7 +283,21 @@ def main():
             ev = dict(model._events); model._events = None
             for a, b, k in STAGES:
                 if a in ev and b in ev: stage[k] = stage.get(k, 0.0) + ev[a].elapsed_time(ev[b])
-        return dev_ms, n_inst, n_cand, stage
+            last = (labels, res)
+        return dev_ms, n_inst, n_cand, stage, last
+
+    def dump(arrays):
+        """--dump-outputs: one float32 / float64 .npy per array (integers up to 2^24 are exact in float32)"""
+        if not args.dump_outputs or rank != 0:
+            return
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in arrays.items():
+            a = np.asarray(a)
+            a = a.astype(np.float64 if a.dtype in (np.float64, np.int64) else np.float32)
+            dumped[0] += a.nbytes
+            assert dumped[0] <= DUMP_LIMIT, "--dump-outputs would exceed %d bytes" % DUMP_LIMIT
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+    dumped = [0]
 
     def time_e2e(model, img, pthr, nthr, steps, warmup=2):
         model._stats = {}
@@ -307,12 +338,14 @@ def main():
     _lib.launch_count(reset=True)
     _lib.profile_enable(True)
     barrier()
-    dev_ms, n_inst, n_cand, stage = time_device(model, x_dev, SHAPE, PROB_THRESH, NMS_THRESH, args.steps)
+    dev_ms, n_inst, n_cand, stage, (labels, res) = time_device(model, x_dev, SHAPE, PROB_THRESH, NMS_THRESH, args.steps)
     launches = _lib.launch_count()
     prof_conv = _lib.profile_get("conv_tc")
     prof_nms = {k: _lib.profile_get("nms2d_" + k) for k in ("frontier", "pairs", "fast", "clip", "tail")}
     _lib.profile_enable(False)
     barrier()
+    dump({"labels_2d": labels, "points_2d": res['points'], "prob_2d": res['prob'], "coord_2d": res['coord']})
+    del labels, res
     (dev_ms_max, _, _), (_, n_total, _) = reduce_max_sum([dev_ms, float(n_inst), 0.0])
     value = n_total / (dev_ms_max / 1000.0)
     e2e = time_e2e(model, img, PROB_THRESH, NMS_THRESH, args.steps)
@@ -358,8 +391,9 @@ def main():
 
     # ------------------------------------------------------------------ configs[2]: 3-D 128x512x512
     if not args.skip_3d:
+        dump3 = None
         try:
-            steps3 = max(2, min(args.steps, 4)); warm3 = 2
+            steps3 = args.steps; warm3 = 2
             cfg3 = bench_data.bench_config_3d(N_RAYS_3D)
             model3 = StarDist3D(cfg3, name=None, basedir=None, weights=bench_data.bench_weights_3d(cfg3))
             vol, _ = bench_data.synthetic_volume(SHAPE_3D, seed=0)
@@ -370,11 +404,15 @@ def main():
             _lib.profile_enable(True)
             l0 = _lib.launch_count()
             barrier()
-            dev_ms3, n_inst3, n_cand3, stage3 = time_device(model3, x3, SHAPE_3D, PROB_THRESH_3D, NMS_THRESH_3D, steps3)
+            dev_ms3, n_inst3, n_cand3, stage3, (labels3, res3) = time_device(model3, x3, SHAPE_3D, PROB_THRESH_3D, NMS_THRESH_3D, steps3)
             launches3 = _lib.launch_count() - l0
             prof_conv3 = _lib.profile_get("conv_tc")
             prof_n3 = {k: _lib.profile_get("nms3d_" + k) for k in ("pretest", "heavy", "heavy_bound", "hulls", "heavy_s4s3s5", "frontier", "paint")}
             _lib.profile_enable(False)
+            if args.dump_outputs:
+                dump3 = {"labels_3d_sample": labels3.reshape(-1)[dump_voxels_3d(labels3.size)],
+                         "points_3d": res3['points'], "prob_3d": res3['prob'], "dist_3d": res3['dist']}
+            del labels3, res3
             barrier()
             (dev3_max, _, _), (_, n3_total, _) = reduce_max_sum([dev_ms3, float(n_inst3), 0.0])
             peak_mem = torch.cuda.max_memory_allocated() / 2 ** 30
@@ -414,6 +452,8 @@ def main():
             torch.cuda.empty_cache()
         except Exception as e:
             if rank == 0: out["error_3d"] = repr(e)[:400]
+        if dump3 is not None:
+            dump(dump3)
         if clocks is None:
             clocks = sampler.stop()
             if rank == 0: out["clocks"] = clocks

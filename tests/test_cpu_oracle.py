@@ -44,18 +44,28 @@ def _hostcheck():
     return ctypes.CDLL(path)
 
 
-@needs_ref
-@pytest.mark.parametrize("n_rays,radius,noise,seed", [(32, 10, .1, 0), (32, 3, .5, 1), (11, 8, .1, 2), (64, 20, .4, 3), (32, 30, .9, 4)])
-def test_clip_sweep_bit_exact_vs_reference_clipper(n_rays, radius, noise, seed):
-    """clip2d.cuh (host build) == vendored Clipper 6.4.2 on fuzzed polygon pairs, float-bit exact"""
+CLIP_CASES = [(32, 10, .1, 0), (32, 3, .5, 1), (11, 8, .1, 2), (64, 20, .4, 3), (32, 30, .9, 4)]
+CLIP_PAIRS = 40000
+
+
+@pytest.mark.parametrize("n_rays,radius,noise,seed", CLIP_CASES)
+def test_clip_sweep_bit_exact_vs_reference_clipper(n_rays, radius, noise, seed, golden_dir):
+    """clip2d.cuh (host build) == vendored Clipper 6.4.2 on fuzzed polygon pairs, float-bit exact on every pair (where
+    oracle/_ref is not built: against the sha256 of the reference's float32 areas, tests/golden/refshim.npz, make_refshim.py)"""
+    import hashlib
     sys.path.insert(0, os.path.join(ROOT, "tests", "tools"))
     import clip_fuzz as cf
     cf.hc = _hostcheck()
-    a, b = cf.make_pairs(40000, n_rays, radius, noise, seed)
-    r, h, st = cf.run(a, b)
+    a, b = cf.make_pairs(CLIP_PAIRS, n_rays, radius, noise, seed)
+    h, st = cf.host(a, b)
     assert np.count_nonzero(st == 2) == 0
-    assert np.array_equal(r.view(np.int32), h.view(np.int32))
-    assert np.count_nonzero(r) > 1000
+    if cf.ref is not None:          # the reference's Clipper built in oracle/_ref
+        r, _, _ = cf.run(a, b)
+        assert np.array_equal(r.view(np.int32), h.view(np.int32))
+    else:
+        want = np.load(os.path.join(golden_dir, "refshim.npz"))["clip/%d/sha256" % seed].tobytes().decode()
+        assert hashlib.sha256(np.ascontiguousarray(h, "<f4").tobytes()).hexdigest() == want
+    assert np.count_nonzero(h) > 1000
 
 
 def test_capi_exports_every_declared_symbol():
@@ -154,12 +164,17 @@ def test_oracle_reproduces_reference_2d_demo_test():
     assert (st.fp, st.tp, st.fn) == demo2d.REFERENCE_TEST_STATS
 
 
-def test_h5lite_reads_the_reference_weight_file():
-    """pure-Python HDF5 subset reader == the frozen fixture (only where /root/reference is mounted)"""
+@pytest.fixture(scope="module")
+def demo_models(tmp_path_factory):
+    """the reference's models/examples/{2D_demo,3D_demo}, rebuilt byte for byte from tests/golden (demo_models.py)"""
+    import demo_models
+    return demo_models.rebuild(str(tmp_path_factory.mktemp("examples")))
+
+
+def test_h5lite_reads_the_reference_weight_file(demo_models):
+    """pure-Python HDF5 subset reader on the reference's 2D_demo weights_best.h5 == the frozen fixture"""
     import sys, os
-    path = "/root/reference/models/examples/2D_demo/weights_best.h5"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not mounted")
+    path = os.path.join(demo_models, "2D_demo", "weights_best.h5")
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
     import demo2d
     from stardist_b200.io import h5lite
@@ -181,19 +196,16 @@ def test_matching_metrics():
     assert (st.fp, st.tp, st.fn) == (0, 1, 0) and abs(st.mean_matched_score - 80 / 120) < 1e-6
 
 
-def test_model_folder_with_keras_checkpoint_loads():
+def test_model_folder_with_keras_checkpoint_loads(demo_models):
     """StarDist2D(None, name, basedir) on a reference model folder: config.json + thresholds.json + weights_best.h5"""
-    import os
-    if not os.path.exists("/root/reference/models/examples/2D_demo/weights_best.h5"):
-        pytest.skip("reference tree not mounted")
     import stardist_b200 as sd
-    m = sd.StarDist2D(None, name='2D_demo', basedir='/root/reference/models/examples')
+    m = sd.StarDist2D(None, name='2D_demo', basedir=demo_models)
     assert tuple(m.config.grid) == (2, 2) and m.config.n_rays == 32
     assert abs(m.thresholds.prob - 0.4861655269131771) < 1e-12 and m.thresholds.nms == 0.5
     assert m.weights['conv2d_1'][0].shape == (3, 3, 1, 32) and m.weights['dist'][0].shape == (1, 1, 128, 32)
     with pytest.raises(ValueError):
         sd.StarDist2D(sd.Config2D(n_rays=16), name=None, basedir=None, weights=m.weights)
-    m3 = sd.StarDist3D(None, name='3D_demo', basedir='/root/reference/models/examples')
+    m3 = sd.StarDist3D(None, name='3D_demo', basedir=demo_models)
     assert m3.config.backbone == 'resnet' and tuple(m3.config.grid) == (1, 2, 2) and m3.config.n_rays == 96
     assert m3._axes_div_by('ZYX') == (1, 2, 2) and m3.weights['conv3d_1'][0].shape == (7, 7, 7, 1, 32)
 
@@ -404,7 +416,7 @@ HOSTFUNC_NMS3D = ["r14_thr02", "r32_noise01_thr01", "r96_aniso_thr03"]
 @pytest.mark.parametrize("name", HOSTFUNC_NMS2D)
 def test_oracle_host_glue_2d_equals_reference_modules(golden_dir, name):
     """oracle/nms_np.py and oracle/geom2d_np.py against the outputs of the reference's OWN nms.py / geom2d.py
-    (tests/golden/hostfuncs.npz, produced by make_hostfuncs.py from /root/reference): dense and sparse 2-D NMS front-ends
+    (tests/golden/hostfuncs.npz, produced by make_hostfuncs.py from the reference's sources): dense and sparse 2-D NMS front-ends
     (points, prob, dist, original indices) bit-equal, dist_to_coord bit-equal (float32)"""
     g = np.load(os.path.join(golden_dir, "hostfuncs.npz"))
     shape, radius, noise, n_rays, grid, pthr, nthr, seed = cases.NMS2D_CASES[name]
@@ -774,21 +786,10 @@ def test_halfspace_volume_is_exact_for_many_rays():
     assert n_checked >= 40
 
 
-def test_volume_stages_equal_the_reference_qhull_functions():
-    """S3 / S4 volumes of the Qhull-free routines (nms3d_pair.cuh, host build of the device headers) against the reference's own
-    qhull_overlap_kernel / qhull_overlap_convex_hulls (stardist3d_impl.cpp:676-735,880-935, compiled unmodified into
-    oracle/_ref/libsdref.so): the float the NMS compares is the same, incl. near-spherical polyhedra with 187 / 256 rays
-    (every facet on the hull -- the case that overflowed the polygon buffer before the scattered re-clip)."""
-    so = os.path.join(ROOT, "tests", "hostcheck", "_build", "libhostcheck.so")
-    sdref = os.path.join(ROOT, "oracle", "_ref", "libsdref.so")
-    if not (os.path.exists(so) and os.path.exists(sdref)):
-        pytest.skip("hostcheck / oracle/_ref not built")
-    hc = ctypes.CDLL(so); ref = ctypes.CDLL(sdref)
-    for f in (ref.sdref_overlap_kernel, ref.sdref_overlap_convex, hc.hc_overlap_kernel, hc.hc_overlap_convex):
-        f.restype = ctypes.c_float
+def overlap_pairs():
+    """polyhedron pairs of test_volume_stages_equal_the_reference_qhull_functions: (n_rays, noise, ctypes arguments, arrays)"""
     P = ctypes.c_void_p
     rng = np.random.default_rng(1)
-    total = equal = 0
     for n_rays, aniso, noise, n_pairs in ((96, (2, 1, 1), 0.2, 60), (187, None, 0.0, 40), (256, None, 0.02, 30), (128, None, 0.05, 30)):
         rays = cases.rays_golden_spiral(n_rays, aniso)
         v = np.ascontiguousarray(rays.vertices, np.float32); f = np.ascontiguousarray(rays.faces, np.int32)
@@ -798,12 +799,27 @@ def test_volume_stages_equal_the_reference_qhull_functions():
             d2 = (10 * rng.uniform(0.8, 1.2) * (1 + noise * rng.uniform(-1, 1, n_rays))).astype(np.float32)
             pv1 = (c1[None] + d1[:, None] * v).astype(np.float32); pv2 = (c2[None] + d2[:, None] * v).astype(np.float32)
             a = (P(pv1.ctypes.data), P(c1.ctypes.data), P(pv2.ctypes.data), P(c2.ctypes.data), P(f.ctypes.data), n_rays, len(f))
-            for want, got in ((ref.sdref_overlap_kernel(*a), hc.hc_overlap_kernel(*a)), (ref.sdref_overlap_convex(*a), hc.hc_overlap_convex(*a[:4], n_rays))):
-                assert (want >= 1e9) == (got >= 1e9) and (want == 0) == (got == 0), (n_rays, want, got)
-                if want < 1e9:
-                    assert abs(want - got) <= 1e-6 * abs(want), (n_rays, noise, want, got)
-                total += 1; equal += int(np.float32(want).view(np.int32) == np.float32(got).view(np.int32))
-    assert equal >= 0.99 * total, (equal, total)
+            yield n_rays, noise, a, (pv1, c1, pv2, c2, f)
+
+
+def test_volume_stages_equal_the_reference_qhull_functions(golden_dir):
+    """S3 / S4 volumes of the Qhull-free routines (nms3d_pair.cuh, host build of the device headers) against the reference's own
+    qhull_overlap_kernel / qhull_overlap_convex_hulls (stardist3d_impl.cpp:676-735,880-935, compiled unmodified into
+    oracle/_ref/libsdref.so; their values: tests/golden/refshim.npz, make_refshim.py): the float the NMS compares is the same,
+    incl. near-spherical polyhedra with 187 / 256 rays (every facet on the hull -- the case that overflowed the polygon buffer
+    before the scattered re-clip)."""
+    hc = _hostcheck()
+    for f in (hc.hc_overlap_kernel, hc.hc_overlap_convex):
+        f.restype = ctypes.c_float
+    ref = np.load(os.path.join(golden_dir, "refshim.npz"))["overlap"]
+    total = equal = 0
+    for i, (n_rays, noise, a, _) in enumerate(overlap_pairs()):
+        for want, got in ((ref[i, 0], hc.hc_overlap_kernel(*a)), (ref[i, 1], hc.hc_overlap_convex(*a[:4], n_rays))):
+            assert (want >= 1e9) == (got >= 1e9) and (want == 0) == (got == 0), (n_rays, want, got)
+            if want < 1e9:
+                assert abs(want - got) <= 1e-6 * abs(want), (n_rays, noise, want, got)
+            total += 1; equal += int(np.float32(want).view(np.int32) == np.float32(got).view(np.int32))
+    assert total == 2 * len(ref) == 320 and equal >= 0.99 * total, (equal, total)
 
 
 def test_ctypes_signatures_match_the_header():
@@ -921,7 +937,7 @@ for k, (name, rays) in enumerate([("cartesian", R3.Rays_Cartesian(8, 5)), ("octo
 print("RESULT " + json.dumps(out))
 '''
     so = os.path.join(ROOT, "tests", "hostcheck", "_build", "libhostcheck.so")
-    if not (os.path.exists(so) and os.path.exists(os.path.join(ROOT, "oracle", "_ref", "stardist3d.so"))):
+    if not (os.path.exists(so) and ref_ext.available()):
         pytest.skip("hostcheck / oracle/_ref not built")
     env = dict(os.environ, OMP_NUM_THREADS="1")
     r = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, env=env, timeout=900)

@@ -3,14 +3,14 @@ inputs -- integer results (survivor indices, polygons' integer centres, label ma
 from the product (cand_from=model) so that the integer post-processing is compared on identical floats; the maps themselves
 are covered by the float-tolerance tests.  The oracle here is the reference's compiled C++ (oracle/_ref) + the numpy glue
 pinned against the reference's Python modules."""
-import os, sys
+import hashlib, json, os, sys
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 import cases
-from oracle import ref_ext, pipeline2d, pipeline3d
+from oracle import ref_ext, nms_np, pipeline2d, pipeline3d
 
 pytestmark = pytest.mark.gpu
 
@@ -91,10 +91,24 @@ def test_volume_3d_equals_oracle(sd):
     model = sd.StarDist3D(cfg, name=None, basedir=None, weights=bench_data.bench_weights_3d(cfg))
     vol, _ = bench_data.synthetic_volume((128, 256, 256), seed=0, cell=(64, 256, 256))
     labels, res = model.predict_instances(vol, prob_thresh=0.7, nms_thresh=0.3)
-    ref_labels, ref = pipeline3d.predict_instances(cfg, rays_from_json(cfg.rays_json), vol, 0.7, 0.3, cand_from=model)
+    rays = rays_from_json(cfg.rays_json)
+    # the reference's 32 MB label volume is too large to replay: tests/golden/at_size_3d.json holds the sha256 of its int32
+    # bytes and its label count; where oracle/_ref is built the reference's volume is compared in full and against the digest
+    golden = json.load(open(os.path.join(ROOT, "tests", "golden", "at_size_3d.json")))
+    digest = lambda a: hashlib.sha256(np.ascontiguousarray(a, np.int32).tobytes()).hexdigest()
+    if ref_ext.built():
+        ref_labels, ref = pipeline3d.predict_instances(cfg, rays, vol, 0.7, 0.3, cand_from=model)
+        assert digest(ref_labels) == golden["labels_sha256"] and ref_labels.max() == golden["n_labels"]
+        assert np.array_equal(labels, ref_labels)
+    else:
+        prob, dist = model._last_maps()
+        proba, dista, points = pipeline3d.candidates(cfg, prob, dist, vol.shape, 0.7)
+        points, probi, disti, _ = nms_np.non_maximum_suppression_3d_sparse(dista, proba, points, rays, nms_thresh=0.3)
+        ref = dict(points=points, prob=probi, dist=disti)
+        assert labels.shape == tuple(golden["shape"]) and labels.max() == golden["n_labels"]
+        assert digest(labels) == golden["labels_sha256"]
     assert len(ref['prob']) > 2000
     assert np.array_equal(res['points'], ref['points']) and np.array_equal(res['prob'], ref['prob']) and np.array_equal(res['dist'], ref['dist'])
-    assert np.array_equal(labels, ref_labels)
 
 
 CLOUDS = [  # shape, noise, n_rays, prob_thresh, nms_thresh, seed, anisotropy, use_bbox, use_kdtree  (tests/tools/nms3d_serial_fuzz.py)

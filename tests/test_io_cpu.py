@@ -1,7 +1,27 @@
 """Host-side formats either side of the path: ImageJ ROI export, TIFF in/out, the command line parser."""
-import ast, hashlib, os, zipfile
+import hashlib, json, os, zipfile
 import numpy as np
 import pytest
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+OBJ_KWARGS = (dict(), dict(single_mesh=False), dict(uv_map=True, scale=(2, 1, 0.5)), dict(scale=0.01))
+
+
+def polyroi_cases():
+    rng = np.random.default_rng(0)
+    for _ in range(25):
+        n = int(rng.integers(3, 40)); xs = rng.uniform(-5, 300, n); ys = rng.uniform(0, 200, n)
+        for sub in (True, False):
+            for pos in (None, 3):
+                yield xs, ys, pos, sub
+
+
+def obj_polys():
+    import stardist_b200 as sd
+    rays = sd.Rays_GoldenSpiral(12)
+    rng = np.random.default_rng(0)
+    return dict(dist=rng.uniform(2, 6, (4, 12)).astype(np.float32), points=rng.integers(5, 40, (4, 3)),
+                rays_vertices=rays.vertices, rays_faces=rays.faces)
 
 
 def test_polyroi_bytes_golden_and_reference():
@@ -10,19 +30,10 @@ def test_polyroi_bytes_golden_and_reference():
     b = bytes(rois.polyroi_bytearray(x, y, pos=2, subpixel=True))
     assert len(b) == 112 and b[:4] == b"Iout"
     assert hashlib.sha256(b).hexdigest() == "9e394be9b5d3ae592c63d1bd595a585848eff9eca31af44bf83dc8026b2b4719"
-    ref_src = "/root/reference/stardist/utils.py"
-    if not os.path.exists(ref_src):
-        return
-    # the reference's function, compiled in isolation (its module imports csbdeep / skimage, which are not installed)
-    fn = [n for n in ast.parse(open(ref_src).read()).body if isinstance(n, ast.FunctionDef) and n.name == "polyroi_bytearray"][0]
-    ns = {"np": np}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), "ref_utils", "exec"), ns)
-    rng = np.random.default_rng(0)
-    for _ in range(25):
-        n = int(rng.integers(3, 40)); xs = rng.uniform(-5, 300, n); ys = rng.uniform(0, 200, n)
-        for sub in (True, False):
-            for pos in (None, 3):
-                assert bytes(rois.polyroi_bytearray(xs, ys, pos=pos, subpixel=sub)) == bytes(ns["polyroi_bytearray"](xs, ys, pos=pos, subpixel=sub))
+    # the reference's own function on the same inputs: tests/golden/io_ref.json (make_io_ref.py)
+    want = json.load(open(os.path.join(GOLDEN, "io_ref.json")))["polyroi_bytearray"]
+    assert [hashlib.sha256(bytes(rois.polyroi_bytearray(xs, ys, pos=pos, subpixel=sub))).hexdigest()
+            for xs, ys, pos, sub in polyroi_cases()] == want
 
 
 def test_export_imagej_rois_and_tiff_roundtrip(tmp_path):
@@ -51,23 +62,13 @@ def test_cli_parser():
 
 
 def test_export_to_obj_file3D(tmp_path):
-    """text identical to stardist/geometry/geom3d.py:277-347 (compiled in isolation where the reference tree is mounted)"""
-    import stardist_b200 as sd
+    """text identical to stardist/geometry/geom3d.py:277-347 (its output digests: tests/golden/io_ref.json)"""
     from stardist_b200.io import obj
-    rays = sd.Rays_GoldenSpiral(12)
-    rng = np.random.default_rng(0)
-    polys = dict(dist=rng.uniform(2, 6, (4, 12)).astype(np.float32), points=rng.integers(5, 40, (4, 3)),
-                 rays_vertices=rays.vertices, rays_faces=rays.faces)
+    polys = obj_polys()
     text = obj.export_to_obj_file3D(polys, fname=str(tmp_path / "m.obj"))
     assert open(tmp_path / "m.obj").read() == text
-    assert text.count("\nv ") + text.startswith("v ") == 4 * 12 and text.count("f ") == 4 * len(rays.faces) and text.startswith("o poly_0\n")
+    assert text.count("\nv ") + text.startswith("v ") == 4 * 12 and text.count("f ") == 4 * len(polys["rays_faces"]) and text.startswith("o poly_0\n")
     with pytest.raises(ValueError):
         obj.export_to_obj_file3D(dict(dist=polys["dist"]))
-    ref_src = "/root/reference/stardist/geometry/geom3d.py"
-    if not os.path.exists(ref_src):
-        return
-    fns = [n for n in ast.parse(open(ref_src).read()).body if isinstance(n, ast.FunctionDef) and n.name in ("dist_to_coord3D", "export_to_obj_file3D")]
-    ns = {"np": np, "tqdm": (lambda x: x)}
-    exec(compile(ast.Module(body=fns, type_ignores=[]), "ref_geom3d", "exec"), ns)
-    for kw in (dict(), dict(single_mesh=False), dict(uv_map=True, scale=(2, 1, 0.5)), dict(scale=0.01)):
-        assert obj.export_to_obj_file3D(polys, **kw) == ns["export_to_obj_file3D"](dict(polys), **kw)
+    want = json.load(open(os.path.join(GOLDEN, "io_ref.json")))["export_to_obj_file3D"]
+    assert [hashlib.sha256(obj.export_to_obj_file3D(polys, **kw).encode()).hexdigest() for kw in OBJ_KWARGS] == want

@@ -2,7 +2,8 @@
 Usage: python tests/tools/clip_fuzz.py [n_pairs] [n_rays] [radius] [noise] [seed]"""
 import ctypes, sys, numpy as np, os
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-ref = ctypes.CDLL(os.path.join(ROOT, "oracle/_ref/libsdref.so"))
+REF_SO = os.path.join(ROOT, "oracle/_ref/libsdref.so")
+ref = ctypes.CDLL(REF_SO) if os.path.exists(REF_SO) else None      # built only where the reference's sources are
 hc = ctypes.CDLL(os.path.join(ROOT, "tests/hostcheck/_build/libhostcheck.so"))
 
 def make_pairs(n_pairs, n_rays, radius, noise, seed, span=None):
@@ -18,14 +19,21 @@ def make_pairs(n_pairs, n_rays, radius, noise, seed, span=None):
     cb = (ca + rng.integers(-int(sp), int(sp) + 1, (n_pairs, 2))).astype(np.float32)
     return polys(ca), polys(cb)
 
+def host(a, b):
+    n_pairs, n = a.shape[:2]
+    a32 = np.ascontiguousarray(a, np.int32); b32 = np.ascontiguousarray(b, np.int32)
+    h = np.zeros(n_pairs, np.float32); st = np.zeros(n_pairs, np.int32)
+    P = ctypes.c_void_p
+    hc.hc_clip_area_batch(P(a32.ctypes.data), P(b32.ctypes.data), n_pairs, n, P(h.ctypes.data), P(st.ctypes.data))
+    return h, st
+
 def run(a, b):
     n_pairs, n = a.shape[:2]
     a64 = np.ascontiguousarray(a, np.int64); b64 = np.ascontiguousarray(b, np.int64)
-    a32 = np.ascontiguousarray(a, np.int32); b32 = np.ascontiguousarray(b, np.int32)
-    r = np.zeros(n_pairs, np.float32); h = np.zeros(n_pairs, np.float32); st = np.zeros(n_pairs, np.int32)
+    r = np.zeros(n_pairs, np.float32)
     P = ctypes.c_void_p
     ref.sdref_clip_area_batch(P(a64.ctypes.data), P(b64.ctypes.data), n_pairs, n, P(r.ctypes.data))
-    hc.hc_clip_area_batch(P(a32.ctypes.data), P(b32.ctypes.data), n_pairs, n, P(h.ctypes.data), P(st.ctypes.data))
+    h, st = host(a, b)
     return r, h, st
 
 def paths_ref(a, b):
